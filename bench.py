@@ -16,6 +16,8 @@ Contract (one JSON line on stdout from rank 0):
            timed on this host on a bounded sample
 
 `--impl reference` times the reference's CPU implementation alone (rank 0 only).
+`--dump-outputs DIR` (one GPU) writes what the timed steps left on the device, a fixed sample of cells, as DIR/*.npy: two
+builds run with the same arguments can be compared output for output (dump_outputs below).
 A "step" is one LBM_timestep of the whole lattice.  Workload at every N: 512^3 cells per GPU (config 5 of
 BASELINE.json, weak scaling; slabs stacked along z), mixture rho = phi = 1 with kBT = 1e-5, alpha0 = 1.5.
 """
@@ -66,6 +68,9 @@ def parse():
     ap.add_argument("--e2e-intervals", type=int, default=3, help="restart -> steps -> frame intervals of the pipelined e2e leg")
     ap.add_argument("--cpu-size", type=int, default=128, help="edge of the CPU arm's sample box (128^3: 2.6 GB, out of L3)")
     ap.add_argument("--cpu-steps", type=int, default=0, help="0 = sized for ~10-20 s")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU: after the timed steps write f, g (populations) and the 22 hydrovs fields at a fixed seeded sample of "
+                         "cells as DIR/{f,g,hydrovars}.npy (float64)")
     return ap.parse_args()
 
 
@@ -161,8 +166,8 @@ def host_cores():
 
 
 def _cpu_oracle(size, kbt):
+    # the checkers are built by __graft_entry__.build(); the bench only loads them, so it can run from a read-only tree
     from oracle import oracle as om
-    om.build()
     prm = dict(kBT=kbt, tau_f=PARAMS["tau_f"], tau_g=PARAMS["tau_g"], alpha0=PARAMS["alpha0"], alpha1=0.0, kappa=PARAMS["kappa"])
     if om.RefOracle.available(fast=True):
         O = om.RefOracle(size, size, size, fast=True)
@@ -238,6 +243,8 @@ def run_b200(a):
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (there is no CPU fallback for the b200 arm)")
+    if a.dump_outputs and world > 1:
+        raise SystemExit("bench.py --dump-outputs: one GPU only")
     torch.cuda.set_device(local)
     numa = bind_to_gpu_numa_node(local) if world > 1 else None
     if world > 1:
@@ -327,6 +334,8 @@ def run_b200(a):
         mt = torch.tensor(mass, device="cuda", dtype=torch.float64)
         dist.all_reduce(mt, op=dist.ReduceOp.SUM)
         mass = [float(v) for v in mt.tolist()]
+    if a.dump_outputs:  # before anything steps the lattice again
+        dump_outputs(b, np, torch, lat, a.dump_outputs)
 
     # ---- dominant kernel alone: per-kernel events inside the library, same step count -------------------
     roofline = None
@@ -396,6 +405,37 @@ def run_b200(a):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_CELLS = 1 << 16  # cells written by --dump-outputs: 60 float64 per cell, 31.5 MB in all
+
+
+def dump_outputs(b, np, torch, lat, out_dir):
+    """What a caller of the timed steps receives -- the populations f, g (fold, gold) and the 22 hydrovs fields -- at DUMP_CELLS
+    cells drawn with a fixed seed (every cell of a smaller box), written as float64 arrays (components, cells) to
+    out_dir/{f,g,hydrovars}.npy.  The fields are copied device to device and sampled there: at 512^3 the full populations
+    are 40.8 GB."""
+    from bflbm_b200.lattice import _check
+    n = lat.nx * lat.ny * lat.nz
+    cells = np.arange(n) if n <= DUMP_CELLS else np.sort(np.random.default_rng(0).choice(n, DUMP_CELLS, replace=False))
+    dev = torch.device("cuda", lat.device)
+    cells = torch.from_numpy(cells).to(dev)
+    f = torch.empty((b.NVEL, n), dtype=torch.float64, device=dev)
+    g = torch.empty_like(f)
+    _check(lat.lib.bflbm_get_populations_device(lat.h, f.data_ptr(), g.data_ptr()))
+    out = {"f": f[:, cells].cpu().numpy(), "g": g[:, cells].cpu().numpy()}
+    # beside the lattice (91.4 GB at 512^3) there are f and g together (40.8 GB), then hydrovs alone (23.6 GB); the cache is
+    # emptied in between and at the end, so the library's later allocations (the e2e leg's staging area) find the memory free
+    del f, g
+    torch.cuda.empty_cache()
+    h = torch.empty((b.NHYDRO, n), dtype=torch.float64, device=dev)
+    _check(lat.lib.bflbm_get_hydrovars_device(lat.h, h.data_ptr()))
+    out["hydrovars"] = h[:, cells].cpu().numpy()
+    del h
+    torch.cuda.empty_cache()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def slab_parity_check(b, np, torch, dist, local, want):
@@ -568,6 +608,8 @@ def run_e2e(a, b, np, torch, lat, stepper, world, cells, cells_local):
 
 if __name__ == "__main__":
     args = parse()
+    if args.impl == "reference" and args.dump_outputs:
+        raise SystemExit("bench.py --dump-outputs: the b200 arm only")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -1,9 +1,12 @@
 """bench.py's output contract on a CPU-only box: the reference arm (the reference's own LBM_timestep on the host cores)
 prints ONE JSON line with the keys the driver reads; the GPU arm refuses to run without a GPU instead of falling back."""
+import importlib.util
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -29,6 +32,30 @@ def test_gpu_arm_has_no_cpu_fallback():
         pytest.skip("GPU present")
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"], capture_output=True, text=True, timeout=600)
     assert r.returncode != 0 and "no CUDA device" in (r.stderr + r.stdout)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_state_after_warmup_plus_timed_steps(bflbm, tmp_path):
+    """--dump-outputs writes the fields of the timed lattice after exactly W + K steps: the noise is keyed by the step number,
+    so one step more or less gives other populations.  A 16^3 box is smaller than the sample: every cell, in order."""
+    import numpy as np
+    out = tmp_path / "dump"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--nx", "16", "--ny", "16", "--nz", "16", "--steps", "3", "--warmup", "2",
+                        "--no-e2e", "--no-cpu", "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr
+    assert json.loads(r.stdout.splitlines()[-1])["steps"] == 3
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    with bflbm.Lattice(16, 16, 16, params=bflbm.Params(**bench.PARAMS)) as lat:
+        lat.set_algorithm("fused")
+        lat.init_mixture()
+        lat.step(5)
+        f, g = lat.populations()
+        want = {"f": f, "g": g, "hydrovars": lat.hydrovars()}
+    for name, w in want.items():
+        got = np.load(out / f"{name}.npy")
+        assert got.dtype == np.float64 and np.array_equal(got, w.reshape(w.shape[0], -1)), name
 
 
 class _FakeLat:

@@ -40,7 +40,7 @@ def test_flow_coefficients_match_the_reference_functions(bflbm, oracle_mod):
 
 def test_fixture_is_the_reference_fit(oracle_mod):
     if not oracle_mod.RefFit.available():
-        pytest.skip("oracle/_ref/libbflbm_ref_fit.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libbflbm_ref_fit.so not built from the original project's source tree: make -C oracle ref REFERENCE=<that tree>")
     import importlib.util
     spec = importlib.util.spec_from_file_location("make_fit_golden", os.path.join(HERE, "golden", "make_fit_golden.py"))
     G = importlib.util.module_from_spec(spec)

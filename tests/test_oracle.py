@@ -74,7 +74,7 @@ def test_port_analytic_inits_match_golden(oracle_mod, init, arg, shape):
 
 def test_port_matches_reference_headers_bitwise(oracle_mod):
     if not oracle_mod.RefOracle.available():
-        pytest.skip("oracle/_ref not built here (needs /root/reference)")
+        pytest.skip("oracle/_ref not built from the original project's source tree: make -C oracle ref REFERENCE=<that tree>")
     rng = np.random.default_rng(3)
     shape = (7, 9, 8)
     for params in (dict(kBT=0.0, tau_f=0.5, tau_g=0.5, alpha0=4.0, alpha1=0.0, kappa=4.0),
@@ -164,7 +164,7 @@ def test_port_reference_state_noise_matches_ref_build_bitwise(oracle_mod):
     restatement of that branch is pinned bit for bit, with injected normals, general relaxation times and an equilibrium state
     displaced by (2, -1, 3) cells so that every component of the integer shift is non-zero."""
     if not oracle_mod.RefOracle.available(ref_state=True):
-        pytest.skip("oracle/_ref/libbflbm_ref_refstate.so not built (needs /root/reference)")
+        pytest.skip("oracle/_ref/libbflbm_ref_refstate.so not built from the original project's source tree: make -C oracle ref REFERENCE=<that tree>")
     shape = (10, 12, 14)
     rng = np.random.default_rng(5)
     prm = dict(kBT=2e-5, tau_f=0.7, tau_g=0.6, alpha0=1.5, alpha1=0.0, kappa=0.1)
