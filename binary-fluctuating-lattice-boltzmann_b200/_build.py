@@ -36,13 +36,15 @@ SF_LIB = os.path.join(HERE, "libbflbm_sf.so")
 
 
 def build_sf(force: bool = False) -> str:
-    """Compile csrc/sf.cu (on-GPU structure-factor accumulator, cuFFT) into libbflbm_sf.so on top of libbflbm.so."""
+    """Compile csrc/sf.cu and csrc/sf_slab.cu (on-GPU structure-factor accumulators, cuFFT) into libbflbm_sf.so on top of
+    libbflbm.so."""
     build()
-    src = os.path.join(CSRC, "sf.cu")
-    deps = [src, LIB, os.path.join(HERE, "..", "include", "bflbm_sf.h")]
+    srcs = [os.path.join(CSRC, s) for s in ("sf.cu", "sf_slab.cu")]
+    deps = srcs + [LIB, os.path.join(CSRC, "sf_common.cuh")] + \
+        [os.path.join(HERE, "..", "include", h) for h in ("bflbm_sf.h", "bflbm_sf_slab.h")]
     if not force and os.path.exists(SF_LIB) and all(os.path.getmtime(d) <= os.path.getmtime(SF_LIB) for d in deps):
         return SF_LIB
-    cmd = [nvcc()] + NVCC_FLAGS + [src, "-o", SF_LIB, "-L" + HERE, "-lbflbm", "-lcufft", "-Xlinker", "-rpath,$ORIGIN"]
+    cmd = [nvcc()] + NVCC_FLAGS + srcs + ["-o", SF_LIB, "-L" + HERE, "-lbflbm", "-lcufft", "-Xlinker", "-rpath,$ORIGIN"]
     subprocess.run(cmd, check=True)
     return SF_LIB
 

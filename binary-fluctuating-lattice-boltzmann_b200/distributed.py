@@ -82,15 +82,24 @@ def _device_tensor(ptr: int, n: int, device):
 class EmulatedSlabs:
     """P slabs of one box held by ONE process on ONE GPU, stepped in lock-step with device-to-device copies in
     place of the NCCL messages.  Exercises exactly the library path a multi-GPU run takes (bflbm_create_slab,
-    step_begin / step_end, halo buffers); used by the single-GPU tests of the slab logic."""
+    step_begin / step_end, halo buffers); used by the single-GPU tests of the slab logic.  structure_factor.SlabStructureFactor
+    accepts it in place of a SlabLattice and moves its all-to-all blocks by device copies as well.
 
-    def __init__(self, nx, ny, nz, nslabs, params: Params | None = None, device: int = 0, brick_lz: int = 0, peer: bool = False):
+    zsplit: optional first planes of the slabs plus nz (nslabs + 1 entries) for an uneven cut; default slab_bounds."""
+
+    def __init__(self, nx, ny, nz, nslabs, params: Params | None = None, device: int = 0, brick_lz: int = 0, peer: bool = False,
+                 zsplit=None):
         import torch
         self.world, self.nz_global = nslabs, nz
         self.peer = peer
         self.device = torch.device("cuda", device)
         self.stream = torch.cuda.Stream(device=self.device)
-        self.bounds = [slab_bounds(nz, nslabs, r) for r in range(nslabs)]
+        if zsplit is None:
+            self.bounds = [slab_bounds(nz, nslabs, r) for r in range(nslabs)]
+        else:
+            if len(zsplit) != nslabs + 1 or zsplit[0] != 0 or zsplit[-1] != nz or any(b - a < 2 for a, b in zip(zsplit, zsplit[1:])):
+                raise ValueError(f"zsplit {list(zsplit)}: need 0 = z_0 < z_1 < ... < z_{nslabs} = {nz}, >= 2 planes per slab")
+            self.bounds = [(int(a), int(b - a)) for a, b in zip(zsplit, zsplit[1:])]
         self.lats = [Lattice(nx, ny, nz, params=params, device=device, slab=b) for b in self.bounds]
         for lat in self.lats:
             lat.set_stream(self.stream.cuda_stream)
