@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <algorithm>
+#include <array>
 #include <map>
 #include <new>
 #include <string>
@@ -121,6 +122,12 @@ struct bflbm_lattice {
   int graph_step_off = 0, graph_bump = 0;
   bool wrapped_in_fold = false;
   bool ghosts_stale = false;  // two-pass steps leave the ghost planes of X and R behind
+
+  // what the last step launched (bflbm_debug_last_step), written on the host where the step kernel is launched; a graph
+  // keeps the record of its capture, which run_graph_chunk restores on every replay
+  std::array<int, BFLBM_LAST_STEP_FIELDS> last_step{};
+  bool last_step_set = false;
+  std::map<long long, std::array<int, BFLBM_LAST_STEP_FIELDS>> graph_last_step;
 
   // USE_REF_STATE noise (LBM_binary.H:12, 92-107; bflbm_set_reference_state): equilibrium profiles [rho_eq | phi_eq | rhot_eq], the
   // centre of mass of rho_eq, and the integer shift (com - com_ref) the device recomputes after every step
@@ -456,6 +463,13 @@ int ensure_full_R(bflbm_lattice* h) {
   return 0;
 }
 
+// the fields of bflbm_debug_last_step, in its order (include/bflbm.h)
+void record_step(bflbm_lattice* h, int algo, int threads, int tile_x, int tile_y, int lz, int nbx, int nby, int nbz, bool full,
+                 bool rate1, bool noise, bool staged_from_e, int schedule) {
+  h->last_step = {algo, threads, tile_x, tile_y, lz, nbx, nby, nbz, full, rate1, noise, staged_from_e, schedule, h->in_graph_capture};
+  h->last_step_set = true;
+}
+
 // rows: 0 = every brick row, 1 = the first and the last row (two z-blocks), 2 = rows 1 .. bz-2
 template <bool NOISE, bool R1, bool FU>
 int launch_fused_v(bflbm_lattice* h, int rows, cudaStream_t st) {
@@ -463,6 +477,7 @@ int launch_fused_v(bflbm_lattice* h, int rows, cudaStream_t st) {
   const dim3 grid(B.bx, B.by, rows == 0 ? B.bz : (rows == 1 ? 2 : B.bz - 2)), block(B.tx, B.ty);
   const int bz0 = rows == 2 ? 1 : 0, two_ends = rows == 1;
   const double2* Ein = (h->e_valid && h->fold_in_staging) ? h->E[h->ecur] : nullptr;
+  record_step(h, 0, B.tx * B.ty, B.tx, B.ty, B.lz, B.bx, B.by, B.bz, FU, R1, NOISE, Ein != nullptr, rows != 0 ? 2 : (h->whole_box ? 0 : 1));
   double2* Eout = h->E[1 - h->ecur];
   const PopBases XB = make_pop_bases(h->G, h->X[h->cur], h->X[1 - h->cur]);
   // inside a graph capture the step is (device counter) + (offset in the chunk); otherwise it is passed by value
@@ -499,6 +514,7 @@ int step_local(bflbm_lattice* h, bool pack = true) {
     const long long* sdev = h->in_graph_capture ? h->d_step : nullptr;
     const bool rate1 = h->rate1_fast_path && h->dp.rate_f == 1. && h->dp.rate_g == 1.;
     const dim3 grid = cell_grid(h, h->G.nzl);
+    record_step(h, 1, h->block.x * h->block.y, h->block.x, h->block.y, 1, grid.x, grid.y, grid.z, false, rate1, noise, false, 0);
 #define BFLBM_TP(N, R1) k_step_twopass<N, R1><<<grid, h->block, 0, h->stream>>>(h->G, h->dp, step, sdev, h->X[h->cur], h->X[1 - h->cur], h->R, rs_of(h))
     if (noise) { if (rate1) BFLBM_TP(true, true); else BFLBM_TP(true, false); }
     else       { if (rate1) BFLBM_TP(false, true); else BFLBM_TP(false, false); }
@@ -593,6 +609,7 @@ int run_graph_chunk(bflbm_lattice* h, int K) {
     h->in_graph_capture = false;
     h->graph_bump = 0;
     h->graph_nodes[key] = h->launches - launches0;
+    h->graph_last_step[key] = h->last_step;
     h->launches = launches0;
     const cudaError_t e = cudaStreamEndCapture(h->stream, &g);
     if (rc || e != cudaSuccess || !g) {
@@ -614,6 +631,8 @@ int run_graph_chunk(bflbm_lattice* h, int K) {
   }
   CU(cudaGraphLaunch(it->second, h->stream));
   h->launches += h->graph_nodes[key];
+  h->last_step = h->graph_last_step[key];
+  h->last_step_set = true;
   h->step += K;
   h->d_step_host += K;
   if (h->algo == 0) {
@@ -1661,6 +1680,14 @@ int bflbm_debug_philox(const unsigned int ctr[4], const unsigned int key[2], uns
   cudaFree(d);
   if (e != cudaSuccess) return fail(BFLBM_ERR_CUDA, "philox test: %s", cudaGetErrorString(e));
   out[0] = r.x; out[1] = r.y; out[2] = r.z; out[3] = r.w;
+  return 0;
+}
+
+int bflbm_debug_last_step(const bflbm_lattice* h, int out[BFLBM_LAST_STEP_FIELDS]) {
+  CHECK_H(h);
+  if (!out) return fail(BFLBM_ERR_ARG, "null output");
+  if (!h->last_step_set) return fail(BFLBM_ERR_STATE, "no step has been launched yet");
+  std::copy(h->last_step.begin(), h->last_step.end(), out);
   return 0;
 }
 

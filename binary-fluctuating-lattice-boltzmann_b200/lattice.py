@@ -24,6 +24,11 @@ NVEL, NHYDRO, NHYDRO_BAR, NNORMALS = 19, 22, 9, 33
 VARIABLE_NAMES = ["rho", "phi", "ufx", "ufy", "ufz", "p_bulk", "ugx", "ugy", "ugz", "afx", "afy", "afz",
                   "agx", "agy", "agz", "ubx", "uby", "ubz", "nfbarx", "ngbarx", "ufbarx", "ugbarx"]
 
+#: fields of bflbm_debug_last_step, in its order (include/bflbm.h): algorithm 0 fused / 1 two-pass; fold_source 1 = staged from
+#: the extended boxes, 0 = every plane from R; schedule 0 whole box / 1 slab on one stream / 2 slab overlapped
+LAST_STEP_FIELDS = ("algorithm", "threads", "tile_x", "tile_y", "lz", "bx", "by", "bz", "full", "rate1", "noise",
+                    "fold_source", "schedule", "graph")
+
 
 class BflbmError(RuntimeError):
     pass
@@ -122,6 +127,7 @@ def load_library() -> ctypes.CDLL:
         "bflbm_second_moments": (ip, [vp, vp]),
         "bflbm_droplet_covariance": (ip, [vp, vp, vp, vp]),
         "bflbm_debug_philox": (ip, [vp, vp, vp]),
+        "bflbm_debug_last_step": (ip, [vp, vp]),
         "bflbm_debug_normal_statistics": (ip, [ctypes.c_ulonglong, ctypes.c_longlong, ctypes.c_longlong, ip, ip, dp, dp, vp, vp, vp]),
         "bflbm_covariance_from_moments": (ip, [vp, vp, vp, vp]),
         "bflbm_set_reference_state": (ip, [vp, vp, vp, vp]),
@@ -459,6 +465,12 @@ class Lattice:
     @property
     def device_bytes(self) -> int:
         return int(self.lib.bflbm_device_bytes(self.h))
+
+    def last_step(self) -> dict:
+        """Which compiled variant of the step kernel the last step launched (bflbm_debug_last_step): a dict of LAST_STEP_FIELDS."""
+        out = (ctypes.c_int * len(LAST_STEP_FIELDS))()
+        _check(self.lib.bflbm_debug_last_step(self.h, out))
+        return dict(zip(LAST_STEP_FIELDS, (int(v) for v in out)))
 
 
 class MultiLattice:

@@ -293,6 +293,21 @@ size_t bflbm_device_bytes(const bflbm_lattice* h);
 /* Philox4x32-10 block function (test hook for known-answer vectors; runs on the device). */
 int bflbm_debug_philox(const unsigned int ctr[4], const unsigned int key[2], unsigned int out[4]);
 
+/* Which compiled variant the last step launched (test hook; recorded on the host where the step kernel is launched, nothing
+ * runs on the device).  out[14]:
+ *   0  algorithm (0 fused, 1 two-pass)       1  threads per CTA
+ *   2  tile x    3  tile y                    (fused: brick tx, ty; two-pass: block.x, block.y)
+ *   4  planes per CTA                         (fused: brick height lz; two-pass: 1)
+ *   5  6  7  CTAs along x, y, z               (fused: bricks bx, by, bz; two-pass: the grid)
+ *   8  FULL (nx, ny multiples of the fused tile: no partial-tile predicates; 0 for two-pass)
+ *   9  RATE1 (tau_f = tau_g = 1/2 specialisation)   10  NOISE (kBT > 0)
+ *   11 fold source (1: the brick-interior planes are staged from the extended boxes of the step before; 0: every plane from R)
+ *   12 schedule (0 whole box, 1 slab on one stream, 2 slab with the interior rows overlapping the exchange)
+ *   13 replayed from a CUDA graph
+ * BFLBM_ERR_STATE before the first step. */
+#define BFLBM_LAST_STEP_FIELDS 14
+int bflbm_debug_last_step(const bflbm_lattice* h, int out[14]);
+
 /* Deep statistics of the in-kernel Gaussian generator (test hook): the 33 normals of ncells cells over nsteps steps binned on the
  * device.  hist[nbins + 2]: equal bins over [lo, hi), then underflow, overflow; joint[32 * 32]: the two normals of one Box-Muller
  * pair over [-4, 4)^2; moments4: sums of n, n^2, n^3, n^4.  10^10 normals take about a second. */
