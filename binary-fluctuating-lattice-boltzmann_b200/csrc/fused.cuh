@@ -196,11 +196,14 @@ inline PopBases make_pop_bases(const Geom& G, const double* X, double* Xn) {
 // setting): that term vanishes, nothing is kept.  General rates: f_old stays in registers, g_old is parked in shared memory.
 
 // FULL: nx and ny are multiples of the tile, every thread owns a cell (no activity predicates, no divergence code).
-template <bool NOISE, bool RATE1, bool FULL, int NT>
+// REF (instantiated with NOISE only): USE_REF_STATE noise -- the amplitudes come from RS.eq (whole-box profiles) at the cell shifted
+// by RS.shift, read once per CTA so that graph replays see the shift of the step before.  RS is not touched when !REF.
+template <bool NOISE, bool RATE1, bool FULL, int NT, bool REF>
 __global__ void __launch_bounds__(NT, 512 / NT)
 k_step_fused(const __grid_constant__ Geom G, const __grid_constant__ BrickGrid B, const __grid_constant__ DevParams P, long long step_arg,
              const long long* __restrict__ step_dev, const __grid_constant__ PopBases XB, const double2* __restrict__ R,
-             const double2* __restrict__ Ein, double2* __restrict__ E, int bz0, int two_ends) {
+             const double2* __restrict__ Ein, double2* __restrict__ E, int bz0, int two_ends, const __grid_constant__ RefState RS) {
+  static_assert(NOISE || !REF, "the reference state only changes the noise amplitudes");
   // time step of the noise key: by value, plus (launches replayed from a CUDA graph) a counter in device memory that the
   // last kernel of every replayed chunk advances -- the arguments of a captured launch cannot change between replays
   const long long step = step_arg + ((NOISE && step_dev != nullptr) ? *step_dev : 0ll);
@@ -244,6 +247,8 @@ k_step_fused(const __grid_constant__ Geom G, const __grid_constant__ BrickGrid B
   constexpr int STG = 2;  // pl = (tx+2)(ty+2) <= 2*NT for every tile shape used (tx in 8..32, tx*ty = NT >= 128)
   int soff[STG];
   if (tid == 0) nfix = 0;
+  __shared__ int ref_shift[3];
+  if (REF && tid < 3) ref_shift[tid] = RS.shift[tid];
   __syncthreads();
 #pragma unroll
   for (int j = 0; j < STG; ++j) {
@@ -408,6 +413,7 @@ k_step_fused(const __grid_constant__ Geom G, const __grid_constant__ BrickGrid B
           }
         }
         float y3[3], ybf[15];
+        double ref3[3];
         {
           double go[Q];
           // all 38 pulls are issued first; the cell's random numbers -- pure arithmetic on its counter -- are generated
@@ -417,6 +423,11 @@ k_step_fused(const __grid_constant__ Geom G, const __grid_constant__ BrickGrid B
           if (RATE1 || !BFLBM_GENERAL_SEQ) {
 #pragma unroll
             for (int i = 0; i < Q; ++i) fo[i] = ld_off(XB.in[i], off[i]);
+          }
+          if (REF) {  // the three equilibrium values travel with the pulls
+            const long long n = G.plane * G.nz_global, rc = ref_offset(G, ref_shift[0], ref_shift[1], ref_shift[2], x, y, zl);
+#pragma unroll
+            for (int k = 0; k < 3; ++k) ref3[k] = __ldg(RS.eq + k * n + rc);
           }
           constexpr bool Y3_LATE = !RATE1 && BFLBM_Y3_LATE;
           if (!Y3_LATE) {
@@ -453,7 +464,7 @@ k_step_fused(const __grid_constant__ Geom G, const __grid_constant__ BrickGrid B
             for (int i = 0; i < PARK_F; ++i) So[(PARK_G + i) * NT + tid] = fo[i];
           }
         }
-        collide_prepare<NOISE, FMA_NOISE>(P, grho, gphi, y3, mf, mg, C);
+        collide_prepare<NOISE, FMA_NOISE>(P, grho, gphi, y3, mf, mg, C, REF ? ref3 : nullptr);
         if (!F_NORMALS_EARLY) mode_normals<NOISE, 0, TAB>(nk, ybf, Trig);
         collide_species<NOISE, 0, RATE1, !RATE1 && BFLBM_F_MOMENT_SPACE, FMA_NOISE>(P, ybf, C, mf);
       } else {

@@ -78,16 +78,17 @@ int main(int argc, char** argv) {
 
     // ---- fluctuating run on the equilibrium reference state, main_run_job.cpp:214-236 + LBM_binary.H:12, 92-107 -------
     if (noiseSwitch && R.use_ref_state) {
-      if (!L.handle()) throw std::runtime_error("use_ref_state needs ngpus = 1 (the centre of mass of the whole box enters every step)");
       std::printf("Noise switch on\n");
       const PlotfileData Er = read_plotfile(eq_name("rho")), Ep = read_plotfile(eq_name("phi")), Et = read_plotfile(eq_name("rhot"));
       for (const PlotfileData* E : {&Er, &Ep, &Et})
         if (E->nx != nx || E->ny != ny || E->nz != nz || E->ncomp != 1) throw std::runtime_error("equilibrium state does not match the box");
       auto total = [](const std::vector<double>& v) { double s = 0.; for (double x : v) s += x; return s; };
       std::printf("Mass rho_eq = %.15g\nMass phi_eq = %.15g\nMass rhot_eq = %.15g\n", total(Er.data), total(Ep.data), total(Et.data));
-      check(bflbm_set_reference_state(L.handle(), Er.data.data(), Ep.data.data(), Et.data.data()));
+      // one GPU: the whole-box call (two-pass kernels); several: every slab on the brick kernel, centre of mass exchanged per step
+      if (L.handle()) check(bflbm_set_reference_state(L.handle(), Er.data.data(), Ep.data.data(), Et.data.data()));
+      else mcheck(bflbm_multi_set_reference_state(L.multi(), Er.data.data(), Ep.data.data(), Et.data.data()));
       double c[3];
-      check(bflbm_get_reference_com(L.handle(), c));
+      check(bflbm_get_reference_com(bflbm_multi_slab(L.multi(), 0), c));
       std::printf("Center of Mass: (%g,%g,%g)\n", c[0], c[1], c[2]);
     } else if (!noiseSwitch) {
       std::printf("Noise switch off, calculating the equilibrium state solutions...\n");

@@ -49,23 +49,27 @@ __device__ __forceinline__ long long nbr(const CellIdx& I, int i) {
   return I.zpl[1 + S * cz(i)] + I.yrow[1 + S * cy(i)] + I.xs[1 + S * cx(i)];
 }
 
-// USE_REF_STATE noise (LBM_binary.H:12, 92-107; whole-box lattices, thread-per-cell kernels): eq = [rho_eq | phi_eq | rhot_eq],
-// each nx*ny*nz doubles; shift = integer part of (centre of mass - com_ref), recomputed on the device after every step.
+// USE_REF_STATE noise (LBM_binary.H:12, 92-107): eq = [rho_eq | phi_eq | rhot_eq], each nx*ny*nz_global doubles (the WHOLE box,
+// also on a slab); shift = integer part of (centre of mass - com_ref), recomputed on the device after every step.
 struct RefState {
   const double* eq;   // nullptr: the shipped behaviour (current densities)
   const int* shift;
 };
-__device__ __forceinline__ bool ref_densities(const Geom& G, const RefState& RS, int x, int y, int zl, double (&d)[3]) {
-  if (RS.eq == nullptr) return false;
-  int xs = x - RS.shift[0], ys = y - RS.shift[1], zs = zl - RS.shift[2];
-  // single periodic wrap, like the reference (LBM_binary.H:97-102)
+// offset in one eq component of the cell (x, y, global plane z0 + zl) shifted by -s: a single periodic wrap per axis, like the
+// reference (LBM_binary.H:97-102)
+__device__ __forceinline__ long long ref_offset(const Geom& G, int sx, int sy, int sz, int x, int y, int zl) {
+  int xs = x - sx, ys = y - sy, zs = G.z0 + zl - sz;
   if (xs < 0) xs += G.nx;
   if (xs > G.nx - 1) xs -= G.nx;
   if (ys < 0) ys += G.ny;
   if (ys > G.ny - 1) ys -= G.ny;
-  if (zs < 0) zs += G.nzl;
-  if (zs > G.nzl - 1) zs -= G.nzl;
-  const long long n = G.plane * G.nzl, c = (long long)zs * G.plane + (long long)ys * G.nx + xs;
+  if (zs < 0) zs += G.nz_global;
+  if (zs > G.nz_global - 1) zs -= G.nz_global;
+  return (long long)zs * G.plane + (long long)ys * G.nx + xs;
+}
+__device__ __forceinline__ bool ref_densities(const Geom& G, const RefState& RS, int x, int y, int zl, double (&d)[3]) {
+  if (RS.eq == nullptr) return false;
+  const long long n = G.plane * G.nz_global, c = ref_offset(G, RS.shift[0], RS.shift[1], RS.shift[2], x, y, zl);
   d[0] = RS.eq[c];
   d[1] = RS.eq[n + c];
   d[2] = RS.eq[2 * n + c];
@@ -446,6 +450,62 @@ __global__ void __launch_bounds__(256) k_com_shift(const double* __restrict__ pa
     shift[1] = (int)(sh[2][0] / m - cy);
     shift[2] = (int)(sh[3][0] / m - cz);
   }
+}
+// Centre of mass of the brick kernels (reference-state noise on a whole box or a slab): com[4 zg .. 4 zg + 3] = {sum rho, sum rho x,
+// sum rho y, sum rho zg} of every GLOBAL plane zg over R (cell indices as coordinates, like k_diag).  Two levels in a fixed order
+// that depends on (nx, ny) only -- not on the brick grid, the slab cut or the schedule:
+//   k_com_chunks : CTA (chunk, zl) sums the COM_CHUNK cells [chunk * COM_CHUNK, ...) of plane zl, thread t the cells t, t + 256, ...
+//                  of the chunk in order, then a fixed tree -> part[zl][chunk][4]  (many CTAs even for a thin slab of large planes)
+//   k_com_fold_chunks : one thread per global plane adds its chunks in order; planes outside this slab get zeros, so that a sum
+//                  all-reduce of the buffers of all slabs is exact (one contributor per entry) and completes every slab's copy.
+constexpr int COM_THREADS = 256, COM_CHUNK = 32 * COM_THREADS;
+inline int com_chunks(const Geom& G) { return (int)((G.plane + COM_CHUNK - 1) / COM_CHUNK); }
+__global__ void __launch_bounds__(COM_THREADS) k_com_chunks(Geom G, const double2* __restrict__ R, double* __restrict__ part) {
+  __shared__ double sh[4][COM_THREADS];
+  const int zl = blockIdx.y, t = threadIdx.x, c0 = blockIdx.x * COM_CHUNK;
+  const int c1 = (int)min((long long)c0 + COM_CHUNK, G.plane);  // a plane is < 2^29 cells (4 GiB per component, create_common)
+  const double2* Rp = R + (long long)(zl + 1) * G.plane;
+  const double Z = G.z0 + zl;
+  double v[4] = {0., 0., 0., 0.};
+#pragma unroll 8
+  for (int c = c0 + t; c < c1; c += COM_THREADS) {
+    const int y = c / G.nx, x = c - y * G.nx;
+    const double r = __ldg(&Rp[c].x);
+    v[0] += r; v[1] += r * (double)x; v[2] += r * (double)y; v[3] += r * Z;
+  }
+#pragma unroll
+  for (int k = 0; k < 4; ++k) sh[k][t] = v[k];
+  __syncthreads();
+  for (int s = COM_THREADS / 2; s > 0; s >>= 1) {
+    if (t < s) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k) sh[k][t] += sh[k][t + s];
+    }
+    __syncthreads();
+  }
+  if (t < 4) part[((long long)zl * gridDim.x + blockIdx.x) * 4 + t] = sh[t][0];
+}
+__global__ void k_com_fold_chunks(Geom G, const double* __restrict__ part, int nchunk, double* __restrict__ com) {
+  const int zg = blockIdx.x * blockDim.x + threadIdx.x, zl = zg - G.z0;
+  if (zg >= G.nz_global) return;
+  double v[4] = {0., 0., 0., 0.};
+  if (zl >= 0 && zl < G.nzl)
+    for (int j = 0; j < nchunk; ++j)
+#pragma unroll
+      for (int k = 0; k < 4; ++k) v[k] += part[((long long)zl * nchunk + j) * 4 + k];
+#pragma unroll
+  for (int k = 0; k < 4; ++k) com[4ll * zg + k] = v[k];
+}
+// sums the nz plane vectors of k_com_fold_chunks in z order (one thread: the same bits on every slab of a box) and writes
+// shift = (int)(com - c) per axis (C truncation, like the reference's static_cast)
+__global__ void k_com_shift_planes(const double* __restrict__ com, int nz, double cx, double cy, double cz, int* __restrict__ shift) {
+  double s[4] = {0., 0., 0., 0.};
+  for (int z = 0; z < nz; ++z)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) s[k] += com[4ll * z + k];
+  shift[0] = (int)(s[1] / s[0] - cx);
+  shift[1] = (int)(s[2] / s[0] - cy);
+  shift[2] = (int)(s[3] / s[0] - cz);
 }
 __global__ void k_count_nonfinite(const double* __restrict__ a, long long n, unsigned long long* __restrict__ cnt) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;

@@ -8,6 +8,12 @@
 //     for every slab: bflbm_step_end     (device-side wait on the arrival flags, unpack)
 // -- no NCCL, no MPI, no host synchronisation: the host thread only queues launches.  With one device the object is a
 // plain whole-box lattice (CUDA-graph replay for the small boxes).  Everything here goes through the public C ABI.
+//
+// Reference-state noise on slabs (bflbm_multi_set_reference_state): after every bflbm_step_end (and init) each slab holds the
+// per-plane centre-of-mass sums of its own planes in its bflbm_com_buffer; the sum all-reduce the ABI asks for is done here with
+// peer copies of each slab's planes into every other slab's buffer, ordered by cross-device events on per-slab streams that
+// this object owns, then bflbm_com_update.  Still no host synchronisation in the step loop.
+#include <cuda_runtime.h>
 #include <stdio.h>
 #include <string.h>
 #include <new>
@@ -22,6 +28,10 @@ struct bflbm_multi {
   std::vector<int> dev, z0, nzl;
   int nx = 0, ny = 0, nz = 0;
   bool whole = true;
+  // reference-state noise on slabs: per-slab streams (handed to the lattices) and events of the centre-of-mass exchange
+  bool ref = false, initialized = false, copies_in_flight = false;
+  std::vector<cudaStream_t> st;
+  std::vector<cudaEvent_t> ev_com, ev_copied;
 };
 
 namespace {
@@ -48,9 +58,94 @@ const char* bflbm_multi_last_error(void) { return g_merr.c_str(); }
 
 int bflbm_multi_destroy(bflbm_multi* m) {
   if (!m) return 0;
-  for (bflbm_lattice* l : m->L) bflbm_destroy(l);
+  for (bflbm_lattice* l : m->L) bflbm_destroy(l);  // synchronises each lattice's stream first
+  for (size_t r = 0; r < m->st.size(); ++r) {
+    cudaSetDevice(m->dev[r]);
+    cudaEventDestroy(m->ev_com[r]);
+    cudaEventDestroy(m->ev_copied[r]);
+    cudaStreamDestroy(m->st[r]);
+  }
   delete m;
   return 0;
+}
+
+namespace {
+#define MCU(call)                                                                                   \
+  do {                                                                                              \
+    const cudaError_t e_ = (call);                                                                  \
+    if (e_ != cudaSuccess) return mfail(BFLBM_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_)); \
+  } while (0)
+// a slab may overwrite its centre-of-mass buffer (bflbm_step_end, inits) only after every other slab has copied its planes
+int wait_com_copies(bflbm_multi* m) {
+  if (!m->copies_in_flight) return 0;
+  const int P = (int)m->L.size();
+  for (int s = 0; s < P; ++s) {
+    MCU(cudaSetDevice(m->dev[s]));
+    for (int r = 0; r < P; ++r)
+      if (r != s) MCU(cudaStreamWaitEvent(m->st[s], m->ev_copied[r], 0));
+  }
+  m->copies_in_flight = false;
+  return 0;
+}
+// the sum all-reduce of bflbm_com_buffer: slab s's planes [z0_s, z0_s + nzl_s) are its own, everything else is zero, so the sum is
+// a copy of each owner's planes
+int exchange_com(bflbm_multi* m) {
+  const int P = (int)m->L.size();
+  for (int r = 0; r < P; ++r) {
+    MCU(cudaSetDevice(m->dev[r]));
+    MCU(cudaEventRecord(m->ev_com[r], m->st[r]));
+  }
+  for (int r = 0; r < P; ++r) {
+    MCU(cudaSetDevice(m->dev[r]));
+    double* dst = static_cast<double*>(bflbm_com_buffer(m->L[r]));
+    for (int s = 0; s < P; ++s) {
+      if (s == r) continue;
+      const double* src = static_cast<const double*>(bflbm_com_buffer(m->L[s]));
+      MCU(cudaStreamWaitEvent(m->st[r], m->ev_com[s], 0));
+      MCU(cudaMemcpyPeerAsync(dst + 4 * (size_t)m->z0[s], m->dev[r], src + 4 * (size_t)m->z0[s], m->dev[s], 4 * (size_t)m->nzl[s] * sizeof(double),
+                              m->st[r]));
+    }
+    const int rc = bflbm_com_update(m->L[r]);
+    if (rc) return mfail(rc, bflbm_last_error());
+    MCU(cudaEventRecord(m->ev_copied[r], m->st[r]));
+  }
+  m->copies_in_flight = true;
+  return 0;
+}
+// after an init: the slabs' centre of mass
+int after_init(bflbm_multi* m) {
+  m->initialized = true;
+  return (m->ref && !m->whole) ? exchange_com(m) : 0;
+}
+}  // namespace
+
+int bflbm_multi_set_reference_state(bflbm_multi* m, const double* rho_eq, const double* phi_eq, const double* rhot_eq) {
+  MCHECK(m);
+  if (!m->whole && rho_eq && m->st.empty()) {
+    for (size_t r = 0; r < m->L.size(); ++r) {
+      MCU(cudaSetDevice(m->dev[r]));
+      cudaStream_t s = nullptr;
+      cudaEvent_t a = nullptr, b = nullptr;
+      cudaError_t e = cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking);
+      if (e == cudaSuccess) e = cudaEventCreateWithFlags(&a, cudaEventDisableTiming);
+      if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b, cudaEventDisableTiming);
+      if (e != cudaSuccess) {  // the three vectors only ever hold complete triples (bflbm_multi_destroy walks them together)
+        if (b) cudaEventDestroy(b);
+        if (a) cudaEventDestroy(a);
+        if (s) cudaStreamDestroy(s);
+        return mfail(BFLBM_ERR_CUDA, std::string("centre-of-mass stream / events: ") + cudaGetErrorString(e));
+      }
+      m->st.push_back(s);
+      m->ev_com.push_back(a);
+      m->ev_copied.push_back(b);
+      const int rc = bflbm_set_stream(m->L[r], s);
+      if (rc) return mfail(rc, bflbm_last_error());
+    }
+  }
+  if (int rc = wait_com_copies(m)) return rc;
+  FOR_ALL(m, bflbm_set_reference_state(l, rho_eq, phi_eq, rhot_eq));
+  m->ref = rho_eq != nullptr;
+  return (m->ref && m->initialized && !m->whole) ? exchange_com(m) : 0;
 }
 
 int bflbm_multi_create(const bflbm_params* p, int nx, int ny, int nz, int ngpus, const int* devices, int brick_lz, bflbm_multi** out) {
@@ -95,15 +190,24 @@ int bflbm_multi_count(const bflbm_multi* m) { return m ? (int)m->L.size() : 0; }
 bflbm_lattice* bflbm_multi_slab(bflbm_multi* m, int i) { return (m && i >= 0 && i < (int)m->L.size()) ? m->L[i] : nullptr; }
 
 int bflbm_multi_set_params(bflbm_multi* m, const bflbm_params* p) { MCHECK(m); FOR_ALL(m, bflbm_set_params(l, p)); return 0; }
-int bflbm_multi_init_mixture(bflbm_multi* m) { MCHECK(m); FOR_ALL(m, bflbm_init_mixture(l)); return 0; }
-int bflbm_multi_init_stripe(bflbm_multi* m, double frac) { MCHECK(m); FOR_ALL(m, bflbm_init_stripe(l, frac)); return 0; }
-int bflbm_multi_init_droplet(bflbm_multi* m, double radius) { MCHECK(m); FOR_ALL(m, bflbm_init_droplet(l, radius)); return 0; }
+#define MULTI_INIT(call)                          \
+  do {                                            \
+    MCHECK(m);                                    \
+    if (int rc_ = wait_com_copies(m)) return rc_; \
+    FOR_ALL(m, call);                             \
+    return after_init(m);                         \
+  } while (0)
+int bflbm_multi_init_mixture(bflbm_multi* m) { MULTI_INIT(bflbm_init_mixture(l)); }
+int bflbm_multi_init_stripe(bflbm_multi* m, double frac) { MULTI_INIT(bflbm_init_stripe(l, frac)); }
+int bflbm_multi_init_droplet(bflbm_multi* m, double radius) { MULTI_INIT(bflbm_init_droplet(l, radius)); }
+#undef MULTI_INIT
 int bflbm_multi_init_from_populations(bflbm_multi* m, const double* f, const double* g) {
   MCHECK(m);
+  if (int rc = wait_com_copies(m)) return rc;
   // every slab uploads its planes (+ the periodic neighbour planes) and packs its halo message; then all of them unpack
   FOR_ALL(m, bflbm_init_from_global_populations(l, f, g));
   if (!m->whole) FOR_ALL(m, bflbm_halo_refresh_end(l));
-  return 0;
+  return after_init(m);
 }
 
 int bflbm_multi_step(bflbm_multi* m, int nsteps) {
@@ -115,7 +219,10 @@ int bflbm_multi_step(bflbm_multi* m, int nsteps) {
   }
   for (int s = 0; s < nsteps; ++s) {
     FOR_ALL(m, bflbm_step_begin(l));
+    if (int rc = wait_com_copies(m)) return rc;  // bflbm_step_end writes the centre-of-mass planes
     FOR_ALL(m, bflbm_step_end(l));
+    if (m->ref)
+      if (int rc = exchange_com(m)) return rc;
   }
   return 0;
 }

@@ -114,6 +114,33 @@ class EmulatedSlabs:
                 lo, hi = neighbours(self.world, r)
                 lat.peer_connect(0, self.lats[lo])
                 lat.peer_connect(1, self.lats[hi])
+        self.com = None          # reference-state noise: the slabs' centre-of-mass buffers
+        self.initialized = False
+
+    def set_reference_state(self, rho_eq=None, phi_eq=None, rhot_eq=None):
+        """Lattice.set_reference_state on every slab (whole-box arrays); steps and inits then exchange the centre of mass."""
+        self._all("set_reference_state", rho_eq, phi_eq, rhot_eq)
+        if rho_eq is None:
+            self.com = None
+            return
+        n = 4 * self.nz_global
+        self.com = [_device_tensor(lat.com_buffer_pointer(), n, self.device) for lat in self.lats]
+        if self.initialized:
+            self._com_exchange()
+
+    def _com_exchange(self):
+        """the sum all-reduce of the centre-of-mass buffers: every entry has one owner and zeros elsewhere, so device copies of
+        each slab's own planes into the others' buffers give the sum"""
+        import torch
+        if self.com is None:
+            return
+        with torch.cuda.stream(self.stream):
+            for r in range(self.world):
+                for s, (z0, nzl) in enumerate(self.bounds):
+                    if s != r:
+                        self.com[r][4 * z0:4 * (z0 + nzl)].copy_(self.com[s][4 * z0:4 * (z0 + nzl)])
+        for lat in self.lats:
+            lat.com_update()
 
     def close(self):
         for lat in self.lats:
@@ -133,14 +160,19 @@ class EmulatedSlabs:
         for lat in self.lats:
             getattr(lat, name)(*a)
 
+    def _init(self, name, *a):
+        self._all(name, *a)
+        self.initialized = True
+        self._com_exchange()
+
     def init_mixture(self):
-        self._all("init_mixture")
+        self._init("init_mixture")
 
     def init_stripe(self, frac=0.5):
-        self._all("init_stripe", frac)
+        self._init("init_stripe", frac)
 
     def init_droplet(self, radius=0.2):
-        self._all("init_droplet", radius)
+        self._init("init_droplet", radius)
 
     def init_from_global_populations(self, f, g):
         for lat, (z0, nzl) in zip(self.lats, self.bounds):
@@ -151,6 +183,8 @@ class EmulatedSlabs:
         self._exchange()
         for lat in self.lats:
             _check(lat.lib.bflbm_halo_refresh_end(lat.h))
+        self.initialized = True
+        self._com_exchange()
 
     def step(self, n=1):
         for _ in range(int(n)):
@@ -159,6 +193,7 @@ class EmulatedSlabs:
             self._exchange()
             for lat in self.lats:
                 _check(lat.lib.bflbm_step_end(lat.h))
+            self._com_exchange()
 
     def gather(self, name):
         """Concatenates a getter's result over the slabs along z (tuple results element-wise)."""
@@ -190,6 +225,8 @@ class SlabLattice:
         self.send = [_device_tensor(lib.bflbm_halo_send_buffer(h, s), n, self.device) for s in (0, 1)]
         self.recv = [_device_tensor(lib.bflbm_halo_recv_buffer(h, s), n, self.device) for s in (0, 1)]
         self.halo_bytes_per_step = 2 * n * 8
+        self.com = None          # reference-state noise: the centre-of-mass buffer, sum-all-reduced after every step and init
+        self.initialized = False
         # peer mode: neighbours' mailboxes mapped through CUDA IPC; from then on a step needs no collective and no Python
         self.peer = False
         if peer:
@@ -216,20 +253,50 @@ class SlabLattice:
         with torch.cuda.stream(self.stream):
             exchange_ring(self.send[0], self.send[1], self.recv[0], self.recv[1], self.rank, self.world, self.group)
 
+    def set_reference_state(self, rho_eq=None, phi_eq=None, rhot_eq=None):
+        """Lattice.set_reference_state (whole-box arrays on every rank); steps and inits then all-reduce the centre of mass.  In
+        peer mode the halo still travels by peer stores; only the centre of mass uses the collective."""
+        self.lat.set_reference_state(rho_eq, phi_eq, rhot_eq)
+        if rho_eq is None:
+            self.com = None
+            return
+        self.com = _device_tensor(self.lat.com_buffer_pointer(), 4 * self.nz_global, self.device)
+        if self.initialized:
+            self._com_exchange()
+
+    def _com_exchange(self):
+        """sum all-reduce of the per-plane centre-of-mass sums (one owner per entry: the same bits on every rank), then the shift"""
+        import torch
+        import torch.distributed as dist
+        if self.com is None:
+            return
+        if self.world > 1:
+            with torch.cuda.stream(self.stream):
+                dist.all_reduce(self.com, op=dist.ReduceOp.SUM, group=self.group)
+        self.lat.com_update()
+
+    def _initialized(self):
+        self.initialized = True
+        self._com_exchange()
+
     def init_mixture(self):
         self.lat.init_mixture()
+        self._initialized()
 
     def init_stripe(self, frac=0.5):
         self.lat.init_stripe(frac)
+        self._initialized()
 
     def init_droplet(self, radius=0.2):
         self.lat.init_droplet(radius)
+        self._initialized()
 
     def init_from_populations_slab(self, f_ghosted, g_ghosted):
         self.lat.init_from_populations_slab(f_ghosted, g_ghosted)
         _check(self.lat.lib.bflbm_halo_refresh_begin(self.lat.h))
         self._exchange()
         _check(self.lat.lib.bflbm_halo_refresh_end(self.lat.h))
+        self._initialized()
 
     def init_from_staged(self):
         """The staged (ghosted) checkpoint of this slab + the halo refresh: init_from_populations_slab without the host."""
@@ -237,6 +304,7 @@ class SlabLattice:
         _check(self.lat.lib.bflbm_halo_refresh_begin(self.lat.h))
         self._exchange()
         _check(self.lat.lib.bflbm_halo_refresh_end(self.lat.h))
+        self._initialized()
 
     def init_from_global_populations(self, f, g):
         """Convenience for tests: every rank passes the WHOLE box (19, nz, ny, nx) and keeps its slab + ghost planes."""
@@ -245,13 +313,14 @@ class SlabLattice:
 
     def step(self, n=1):
         lib, h = self.lat.lib, self.lat.h
-        if self.peer:  # the whole loop runs inside the library: begin (pack = NVLink stores), end (device-side wait, unpack)
+        if self.peer and self.com is None:  # the whole loop runs inside the library: begin (pack = NVLink stores), end (wait, unpack)
             _check(lib.bflbm_step_slab(h, int(n)))
             return
         for _ in range(int(n)):
             _check(lib.bflbm_step_begin(h))
             self._exchange()
             _check(lib.bflbm_step_end(h))
+            self._com_exchange()
 
     def host_checkpoint(self):
         """bench.py helper (untimed): this slab's populations as a ghosted host checkpoint, (2, 19, nz_local + 2, ny, nx), pinned

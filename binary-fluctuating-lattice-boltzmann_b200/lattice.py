@@ -136,6 +136,11 @@ def load_library() -> ctypes.CDLL:
         "bflbm_debug_fit_coefficients": (ip, [dp, dp, dp, dp, dp, dp, vp]),
         "bflbm_multi_fit_droplet": (ip, [vp, ip, dp, ip, dp, dp, dp, dp, dp, vp, ctypes.POINTER(ip)]),
         "bflbm_get_reference_com": (ip, [vp, vp]),
+        "bflbm_get_reference_shift": (ip, [vp, vp]),
+        "bflbm_com_doubles": (ctypes.c_size_t, [vp]),
+        "bflbm_com_buffer": (vp, [vp]),
+        "bflbm_com_update": (ip, [vp]),
+        "bflbm_multi_set_reference_state": (ip, [vp, vp, vp, vp]),
         "bflbm_init_from_global_populations": (ip, [vp, vp, vp]),
         "bflbm_get_populations_into_global": (ip, [vp, vp, vp]),
         "bflbm_get_hydrovars_into_global": (ip, [vp, vp]),
@@ -332,18 +337,33 @@ class Lattice:
         _check(self.lib.bflbm_init_from_global_populations(self.h, f.ctypes.data, g.ctypes.data))
 
     def set_reference_state(self, rho_eq=None, phi_eq=None, rhot_eq=None):
-        """USE_REF_STATE noise (LBM_binary.H:12, 92-107): amplitudes from these (nz, ny, nx) equilibrium profiles at the
-        COM-shifted cell; None switches back to the shipped behaviour."""
+        """USE_REF_STATE noise (LBM_binary.H:12, 92-107): amplitudes from these equilibrium profiles of the WHOLE box,
+        (nz_global, ny, nx) also for a slab, at the COM-shifted cell; None switches back to the shipped behaviour.  A slab then
+        needs the centre-of-mass exchange after every step and init (com_buffer, com_update; distributed.py does it)."""
         if rho_eq is None:
             _check(self.lib.bflbm_set_reference_state(self.h, None, None, None))
             return
-        a = [_host(v, self.shape, n) for v, n in ((rho_eq, "rho_eq"), (phi_eq, "phi_eq"), (rhot_eq, "rhot_eq"))]
+        shp = (self.nz_global, self.ny, self.nx)
+        a = [_host(v, shp, n) for v, n in ((rho_eq, "rho_eq"), (phi_eq, "phi_eq"), (rhot_eq, "rhot_eq"))]
         _check(self.lib.bflbm_set_reference_state(self.h, a[0].ctypes.data, a[1].ctypes.data, a[2].ctypes.data))
 
     def reference_com(self):
         c = np.empty(3)
         _check(self.lib.bflbm_get_reference_com(self.h, c.ctypes.data))
         return c
+
+    def reference_shift(self):
+        """the integer shift (x, y, z) the next step reads the equilibrium profiles with (synchronises the lattice's stream)"""
+        s = (ctypes.c_int * 3)()
+        _check(self.lib.bflbm_get_reference_shift(self.h, s))
+        return np.array(s, dtype=np.int64)
+
+    def com_buffer_pointer(self) -> int:
+        """device address of the 4 * nz_global doubles of per-plane centre-of-mass sums (slabs: the caller sum-all-reduces them)"""
+        return int(self.lib.bflbm_com_buffer(self.h) or 0)
+
+    def com_update(self):
+        _check(self.lib.bflbm_com_update(self.h))
 
     # -- peer mode (include/bflbm.h): the halo message goes straight into the neighbour's mailbox ----------------
     def peer_ipc_handle(self) -> bytes:
@@ -533,6 +553,20 @@ class MultiLattice:
         f = _host(f, (NVEL,) + self.shape, "f")
         g = _host(g, (NVEL,) + self.shape, "g")
         self._mcheck(self.lib.bflbm_multi_init_from_populations(self.h, f.ctypes.data, g.ctypes.data))
+
+    def set_reference_state(self, rho_eq=None, phi_eq=None, rhot_eq=None):
+        """Lattice.set_reference_state on every slab (whole-box arrays); steps and inits then exchange the centre of mass"""
+        if rho_eq is None:
+            self._mcheck(self.lib.bflbm_multi_set_reference_state(self.h, None, None, None))
+            return
+        a = [_host(v, self.shape, n) for v, n in ((rho_eq, "rho_eq"), (phi_eq, "phi_eq"), (rhot_eq, "rhot_eq"))]
+        self._mcheck(self.lib.bflbm_multi_set_reference_state(self.h, a[0].ctypes.data, a[1].ctypes.data, a[2].ctypes.data))
+
+    def reference_shift(self, slab: int = 0):
+        """the reference-state shift held by slab `slab` (every slab holds the same one)"""
+        s = (ctypes.c_int * 3)()
+        _check(self.lib.bflbm_get_reference_shift(self.lib.bflbm_multi_slab(self.h, int(slab)), s))
+        return np.array(s, dtype=np.int64)
 
     def step(self, n=1):
         self._mcheck(self.lib.bflbm_multi_step(self.h, int(n)))

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Compile csrc/capi.cu with -Xptxas -v and print registers / spills per k_step_fused variant.
+"""Compile csrc/capi.cu with -Xptxas -v and print registers / spills per k_step_fused<NOISE, RATE1, FULL, NT, REF> variant.
 usage: tools/ptxas_report.py [-o out.so] [extra nvcc flags ...]"""
 import os
 import re
@@ -37,6 +37,7 @@ for ln in r.stderr.splitlines():
     if m:
         rows[cur]["regs"] = int(m.group(1))
 for k, v in rows.items():
-    m = re.search(r"k_step_fusedILb([01])ELb([01])ELb([01])ELi(\d+)E", k)
-    if m and m.group(4) == "256":
-        print(f"fused noise={m.group(1)} rate1={m.group(2)} full={m.group(3)}: regs {v.get('regs')} stack {v.get('stack')} spill st/ld {v.get('st')}/{v.get('ld')}")
+    m = re.search(r"k_step_fusedILb([01])ELb([01])ELb([01])ELi(\d+)ELb([01])E", k)
+    if m:
+        print(f"fused noise={m.group(1)} rate1={m.group(2)} full={m.group(3)} nt={m.group(4)} ref={m.group(5)}: regs {v.get('regs')} "
+              f"stack {v.get('stack')} spill st/ld {v.get('st')}/{v.get('ld')}")
