@@ -54,6 +54,9 @@ typedef struct {
    * (centre of mass - com_ref); NULL = the shipped build (current densities) */
   double *rho_eq, *phi_eq, *rhot_eq; /* [n] each */
   double com_ref[3];
+  /* set_ref_shift: the shift the next noise generations use instead of (int)(com - com_ref), so that an oracle on a window of a
+   * larger box can take that box's shift; force_shift = 0 (the default) computes it as the reference does */
+  int force_shift, forced_shift[3];
 } oracle_lattice;
 
 static void init_constants(void) {
@@ -307,6 +310,8 @@ static void thermal_noise_all(oracle_lattice* L, int relative) {
     double com[3];
     center_of_mass(L, L->hb, com);
     for (int d = 0; d < 3; ++d) shift[d] = (int)(relative ? com[d] - L->com_ref[d] : com[d]);
+    if (L->force_shift)
+      for (int d = 0; d < 3; ++d) shift[d] = L->forced_shift[d];
   }
 #ifdef _OPENMP
 #pragma omp parallel for schedule(static)
@@ -453,6 +458,13 @@ void oracle_set_equilibrium(void* h, const double* rho_eq, const double* phi_eq,
   L->rho_eq = (double*)malloc(n * sizeof(double)); L->phi_eq = (double*)malloc(n * sizeof(double)); L->rhot_eq = (double*)malloc(n * sizeof(double));
   memcpy(L->rho_eq, rho_eq, n * sizeof(double)); memcpy(L->phi_eq, phi_eq, n * sizeof(double)); memcpy(L->rhot_eq, rhot_eq, n * sizeof(double));
   center_of_mass(L, L->rho_eq, L->com_ref);
+}
+/* the integer shift (x, y, z) of the reference-state noise for the next noise generations; NULL = computed from the centre of
+ * mass again (test hook: a window of a larger box cannot compute that box's shift) */
+void oracle_set_ref_shift(void* h, const int* shift3) {
+  oracle_lattice* L = (oracle_lattice*)h;
+  L->force_shift = shift3 != NULL;
+  for (int d = 0; d < 3; ++d) L->forced_shift[d] = shift3 ? shift3[d] : 0;
 }
 /* 33 standard normals per cell (cell-major, reference draw order) used by the NEXT noise generation; NULL = zeros */
 void oracle_set_normals(void* h, const double* normals) { ((oracle_lattice*)h)->normals = normals; }

@@ -171,6 +171,13 @@ class PortOracle(_Base):
         assert all(v.shape == self.shape for v in a)
         self._fn("set_equilibrium", None, [_dp, _dp, _dp, _dp])(self.h, _ptr(a[0]), _ptr(a[1]), _ptr(a[2]))
 
+    def set_ref_shift(self, shift):
+        """the integer (x, y, z) shift the next reference-state noise generations read the equilibrium profiles with, in place
+        of (int)(com - com_ref); None (the default) computes it again.  An oracle on a window of a larger box takes that
+        box's shift this way (or shift 0 with profiles cut at window offset - shift)."""
+        s = None if shift is None else (ctypes.c_int * 3)(*(int(v) for v in shift))
+        self._fn("set_ref_shift", None, [_dp, _dp])(self.h, s)
+
     def set_normals(self, normals):
         """normals: (nz, ny, nx, 33) standard normals for the next noise generation, or None."""
         if normals is None:
